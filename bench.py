@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Bench of the SHERF render hot path (ImportanceRenderer.forward + NeRFDecoder + ray marcher) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path over N_gpus novel views of BASELINE.json configs[1]
 (512x512 RenderPeople-shape, 64 samples/ray, one subject / one observation), synthetic seeded inputs.
@@ -10,7 +10,9 @@ granularity (rank r renders view r: the shard of the ray batch it owns), and the
 rendered tiles so that every rank holds all N images (weak scaling: N views on N GPUs).  `--shard tiles` instead
 deals every view's rays to all ranks in interleaved 256-ray tiles with one all-gather per view (the single-view
 latency mode of sherf_b200.dist.render_sharded).
-Prints one JSON line (see README / DESIGN.md "Measurement").
+Prints one JSON line (see README / DESIGN.md "Measurement").  `--dump-outputs DIR` also writes what the last timed step computed as
+DIR/rgb.npy, DIR/depth.npy, DIR/acc.npy (float32, [views, rays, channels]); the inputs are seeded, so two builds run with the same
+arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -65,7 +67,26 @@ def parse():
     ap.add_argument('--shard', default='views', choices=['views', 'tiles'], help='N>1: ray-batch sharding granularity')
     ap.add_argument('--ref-rays', type=int, default=0, help='--impl reference: rays per step (0 = sized for a few minutes in total)')
     ap.add_argument('--ref-dump', default='', help='--impl reference: write the ray indices and the rendered outputs of the last step here (torch.save)')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='write rgb / depth / acc of the last timed step to DIR/<name>.npy (float32, [views, rays, channels])')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    return args
+
+
+DUMP_BYTES_MAX = 64 << 20
+
+
+def dump_outputs(out_dir, images):
+    """images: [views, rays, 5] (rgb, depth, acc), the rendered outputs of one step.  Whole views only: when they exceed DUMP_BYTES_MAX the
+    first views that fit are written."""
+    import numpy as np
+    x = images.detach().float().cpu().numpy()
+    x = x[:max(1, DUMP_BYTES_MAX // (x[0].size * 4))]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, sl in (('rgb', slice(0, 3)), ('depth', slice(3, 4)), ('acc', slice(4, 5))):
+        np.save(os.path.join(out_dir, name + '.npy'), np.ascontiguousarray(x[..., sl]))
 
 
 def peaks():
@@ -195,6 +216,8 @@ def run_reference(args):
         if i >= args.warmup:
             rates.append((rate, dt))
         last = sample
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch.cat([out[0], out[1], out[2]], -1))
     if args.ref_dump:
         torch.save({'idx': idx, 'rgb': out[0], 'depth': out[1], 'acc': out[2], 'u': u, 'kind': kind, 'rate': rates[-1][0], 'seconds': rates[-1][1],
                     'sample': last, 'threads': threads}, args.ref_dump)
@@ -394,6 +417,8 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
+    last_result = [None]                                                              # what the last step of the latest timed() returned
+
     def timed(fn, k):
         """k steps, each bracketed by CUDA events on the launching stream, L2 flushed between steps (outside the events).  The host does not
         wait for a step before it enqueues the next one (one synchronize after the k-th): launches are asynchronous in a real pipeline too,
@@ -405,7 +430,7 @@ def main():
             flush.zero_()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            fn()
+            last_result[0] = fn()
             if i == k - 1:
                 drain_gathers()                                                         # nothing escapes the K timed windows
             e1.record()
@@ -438,6 +463,8 @@ def main():
         clocks.mark()
     overlap_gather[0] = world > 1 and not by_tiles
     ms = timed(step_device, args.steps)
+    # the images of the last timed step: [N, 5] per view rendered here, or [world * N, 5] all-gathered
+    timed_images = torch.cat(last_result[0]).view(-1, N, 5)
     overlap_gather[0] = False
     barrier()
     clk = clocks.stop() if clocks else None
@@ -676,6 +703,8 @@ def main():
                                           'rgb_linf_vs_cuda_path_full_view': float((ours[0] - ref_out[0]).abs().max()),
                                           'acc_linf_vs_cuda_path_full_view': float((ours[2] - ref_out[2]).abs().max()),
                                           'rays_beyond_1e-4': float(((ours[0] - ref_out[0]).abs().amax(-1) > 1e-4).float().mean())}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, timed_images)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,5 +1,5 @@
-"""CPU tests of the checker itself: oracle/port.py against the golden fixtures made from the reference's own code,
-and (only where /root/reference is mounted) against the live shimmed reference on a fresh scene."""
+"""CPU tests of the checker itself: oracle/port.py against the golden fixtures made from the reference's own code: whole renders
+(oracle/gen_golden.py) and single reference functions on fresh inputs (oracle/gen_golden_reference_calls.py)."""
 import os
 
 import numpy as np
@@ -10,6 +10,14 @@ from conftest import GOLDEN_CASES, load_golden
 from sherf_b200 import synthetic as S
 from oracle import port, ref_shim
 from oracle.gen_golden import checksum
+from oracle.gen_golden_reference_calls import sample_index
+
+SAMPLE_IMPORTANCE_ROWS = 50          # rays of each sample_importance case whose reference answer is stored
+
+
+def reference_calls():
+    from conftest import GOLDEN_DIR
+    return np.load(os.path.join(GOLDEN_DIR, 'reference_oracle_calls.npz'))
 
 
 @pytest.mark.parametrize('case', GOLDEN_CASES)
@@ -37,19 +45,17 @@ def test_port_matches_reference_golden(case, smpl_model, smpl_model_t):
     assert np.abs(depth[0].numpy() - g['depth']).max() <= 1e-5
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='reference tree is only mounted in the build container')
 def test_port_matches_live_reference(smpl_model, smpl_model_t):
-    ren, dec = ref_shim.build_reference(smpl_model_t, seed=4)
-    with torch.no_grad():
-        dec.alpha_linear.weight *= 30
-        dec.alpha_linear.bias += 2.0
+    """A fresh scene, not one of the render fixtures, through the reference's forward (weights: the seed-4 set stored with the importance
+    fixture, density head scaled like every fixture)."""
+    g, w = reference_calls(), load_golden('importance_28x20x16p12')['weights']
     scene = S.make_scene(S.SceneSpec(H=20, W=28, samples=12, seed=9, random_global_R=True), smpl_model)
-    ref = ref_shim.render(ren, dec, scene)
-    got = port.render_forward(port.hot_path_state_dict(ren, dec), smpl_model_t, scene)
-    for a, b in zip(ref, got):
-        assert a.shape == b.shape
-        assert float((a - b).abs().max()) <= 1e-5
-    assert float(ref[2].max()) > 0.2          # the body is actually visible
+    assert checksum(scene) == str(g['live/input_sha256'])
+    got = port.render_forward(w, smpl_model_t, scene)
+    for a, b in zip([g['live/rgb'], g['live/depth'], g['live/acc']], got):
+        assert a.shape == tuple(b.shape)
+        assert float(np.abs(a - b.numpy()).max()) <= 1e-5
+    assert float(g['live/acc'].max()) > 0.2          # the body is actually visible
 
 
 def test_port_importance_matches_golden(smpl_model, smpl_model_t):
@@ -71,21 +77,19 @@ def test_port_importance_matches_golden(smpl_model, smpl_model_t):
     assert np.abs(depth[0].numpy() - g['depth']).max() <= 1e-5
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='reference tree is only mounted in the build container')
 def test_port_importance_matches_live_reference(smpl_model, smpl_model_t):
-    ren, dec = ref_shim.build_reference(smpl_model_t, seed=6)
-    with torch.no_grad():
-        dec.alpha_linear.weight *= 30
-        dec.alpha_linear.bias += 2.0
+    """A fresh scene through the reference's repaired coarse + fine pass (oracle/ref_shim.render_importance; weights: the seed-1 set stored with
+    the ragged fixture)."""
+    g, w = reference_calls(), load_golden('ragged_45x38x24_R_white')['weights']
     scene = S.make_scene(S.SceneSpec(H=18, W=22, samples=10, seed=17, white_back=True), smpl_model)
+    assert checksum(scene) == str(g['live_importance/input_sha256'])
     scene['rendering_options']['depth_resolution_importance'] = 7
     u = torch.rand(18 * 22, 7, generator=torch.Generator().manual_seed(5))
-    ref = ref_shim.render_importance(ren, dec, scene, u, return_stages=True)
-    got = port.render_forward(port.hot_path_state_dict(ren, dec), smpl_model_t, scene, return_stages=True, importance_u=u)
-    for a, b in zip(ref[:3], got[:3]):
-        assert a.shape == b.shape
-        assert float((a - b).abs().max()) <= 1e-5
-    assert float((ref[3]['t_fine'] - got[3]['t_fine']).abs().max()) <= 5e-6
+    got = port.render_forward(w, smpl_model_t, scene, return_stages=True, importance_u=u)
+    for a, b in zip([g['live_importance/rgb'], g['live_importance/depth'], g['live_importance/acc']], got[:3]):
+        assert a.shape == tuple(b.shape)
+        assert float(np.abs(a - b.numpy()).max()) <= 1e-5
+    assert float(np.abs(g['live_importance/t_fine'] - got[3]['t_fine'].numpy()).max()) <= 5e-6
 
 
 def test_sample_importance_properties():
@@ -130,12 +134,8 @@ def test_composite_background_and_clamp():
     assert torch.allclose(rgb[1], torch.tensor([0.2, 0.4, 0.6]) * 2 - 1, atol=1e-5)
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='reference tree is only mounted in the build container')
-@pytest.mark.parametrize('S_,SF', [(16, 12), (64, 64), (5, 9)])
-def test_sample_importance_matches_reference_function(S_, SF, smpl_model_t):
-    """port.sample_importance against the reference's OWN sample_importance / sample_pdf (renderer.py:483-542) on random ray-marcher
-    weights, with torch.rand (:526) returning the same draws: identical bins, depths to the last few ulp."""
-    ren, _ = ref_shim.build_reference(smpl_model_t, seed=0)
+def sample_importance_inputs(S_, SF):
+    """300 rays of random ray-marcher weights (every fourth ray all zero) and the uniform draws standing for torch.rand."""
     g = torch.Generator().manual_seed(S_ * 100 + SF)
     n = 300
     near = torch.rand(n, generator=g) + 0.5
@@ -144,23 +144,23 @@ def test_sample_importance_matches_reference_function(S_, SF, smpl_model_t):
     w = torch.rand(n, S_, generator=g) ** 6
     w[::4] = 0
     u = torch.rand(n, SF, generator=g)
-    orig = torch.rand
-    torch.rand = lambda *a, **k: u
-    try:
-        want = ren.sample_importance(depths.view(1, n, S_, 1), w.view(1, n, S_, 1), SF)[0, :, :, 0]
-    finally:
-        torch.rand = orig
+    return near, far, depths, w, u
+
+
+@pytest.mark.parametrize('S_,SF', [(16, 12), (64, 64), (5, 9)])
+def test_sample_importance_matches_reference_function(S_, SF):
+    """port.sample_importance against the reference's OWN sample_importance / sample_pdf (renderer.py:483-542) on random ray-marcher
+    weights, with torch.rand (:526) returning the same draws: identical bins, depths to the last few ulp (the reference's answer is stored
+    for a fixed sample of the rays)."""
+    near, far, depths, w, u = sample_importance_inputs(S_, SF)
+    want = torch.from_numpy(reference_calls()[f'sample_importance/{S_}_{SF}'])
     got, bins = port.sample_importance(depths, w, SF, u)
-    assert float((got - want).abs().max()) <= 1e-6 * float((far - near).max())
+    assert float((got[sample_index(got.shape[0], SAMPLE_IMPORTANCE_ROWS, S_ * 100 + SF)] - want).abs().max()) <= 1e-6 * float((far - near).max())
     assert int(bins.min()) >= 1 and int(bins.max()) <= S_ - 2
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason='reference tree is only mounted in the build container')
-@pytest.mark.parametrize('white', [False, True])
-def test_composite_and_unify_match_reference_functions(white, smpl_model_t):
-    """port.composite == the reference's MipRayMarcher2 (ray_marcher.py:25-64) and port.unify_samples == ImportanceRenderer.unify_samples
-    (renderer.py:446-456) on random colours / densities / depths (incl. sigma = -80 "culled" samples and empty rays)."""
-    ren, _ = ref_shim.build_reference(smpl_model_t, seed=0)
+def composite_inputs():
+    """Random colours / densities / depths, incl. sigma = -80 "culled" samples and empty rays."""
     g = torch.Generator().manual_seed(11)
     n, S1, S2 = 200, 16, 12
     d1 = port.sample_depths(torch.rand(n, generator=g) + 0.5, torch.rand(n, generator=g) + 2.0, S1)
@@ -171,17 +171,27 @@ def test_composite_and_unify_match_reference_functions(white, smpl_model_t):
     s1[::7] = -80.0
     s2[::7] = -80.0
     rays_d = torch.randn(n, 3, generator=g)
-    opts = {'clamp_mode': 'relu', 'white_back': white}
-    ref_rgb, ref_depth, ref_w = ren.ray_marcher(c1[None], s1[None, :, :, None], d1[None, :, :, None], rays_d[None], opts)
+    return d1, d2, c1, c2, s1, s2, rays_d
+
+
+@pytest.mark.parametrize('white', [False, True])
+def test_composite_and_unify_match_reference_functions(white):
+    """port.composite == the reference's MipRayMarcher2 (ray_marcher.py:25-64) and port.unify_samples == ImportanceRenderer.unify_samples
+    (renderer.py:446-456) on random colours / densities / depths (incl. sigma = -80 "culled" samples and empty rays).  unify_samples
+    permutes the concatenated samples: the fixture holds the permutation it applied."""
+    g = reference_calls()
+    d1, d2, c1, c2, s1, s2, rays_d = composite_inputs()
+    ref_rgb, ref_depth, ref_w = (torch.from_numpy(g[f'composite/{int(white)}/{k}']) for k in ('rgb', 'depth', 'weights'))
     rgb, depth, w = port.composite(c1, s1, d1, rays_d, white)
-    assert float((rgb - ref_rgb[0]).abs().max()) <= 1e-6 and float((w - ref_w[0, :, :, 0]).abs().max()) <= 1e-6
-    assert torch.equal(depth, ref_depth[0])
-    ad, ac, as_ = ren.unify_samples(d1[None, :, :, None], c1[None], s1[None, :, :, None], d2[None, :, :, None], c2[None], s2[None, :, :, None])
+    assert float((rgb - ref_rgb).abs().max()) <= 1e-6 and float((w - ref_w).abs().max()) <= 1e-6
+    assert torch.equal(depth, ref_depth)
+    perm = torch.from_numpy(g['unify/permutation']).long()
+    ad, as_ = torch.cat([d1, d2], 1).gather(1, perm), torch.cat([s1, s2], 1).gather(1, perm)
+    ac = torch.cat([c1, c2], 1).gather(1, perm[..., None].expand(-1, -1, 3))
     pd, pc, ps = port.unify_samples(d1, c1, s1, d2, c2, s2)
-    assert torch.equal(pd, ad[0, :, :, 0]) and torch.equal(pc, ac[0]) and torch.equal(ps, as_[0, :, :, 0])
-    ref2 = ren.ray_marcher(ac, as_, ad, rays_d[None], opts)
+    assert torch.equal(pd, ad) and torch.equal(pc, ac) and torch.equal(ps, as_)
     got2 = port.composite(pc, ps, pd, rays_d, white)
-    assert float((got2[0] - ref2[0][0]).abs().max()) <= 1e-6
+    assert float((got2[0] - torch.from_numpy(g[f'composite/{int(white)}/rgb_unified'])).abs().max()) <= 1e-6
 
 
 def test_branch_free_erf_of_the_transformer_kernel():
