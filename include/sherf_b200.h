@@ -399,6 +399,10 @@ SHERF_API float sherf_last_stage_ms(int stage);
 /* Host wall time (microseconds) of the last forward on this thread: 0 launch issue until the survivor-count sync, 1 time blocked in
  * that sync, 2 launch issue of the point stages and the ray march, 3 whole call. */
 SHERF_API float sherf_last_host_us(int part);
+/* Nearest-vertex candidate lists of the last forward on this thread (synchronises the device): out[0] cull candidates of the last
+ * cull, then for the cull grid (out[1..4]) and the canonical grid (out[5..8]): sub-cells with a list, mean and max list length, fraction
+ * of them over the capacity; out[9] the capacity.  Returns SHERF_OK, or SHERF_E_INVALID when the last forward built no lists. */
+SHERF_API int sherf_nn_list_stats(double* out);
 
 #ifdef __cplusplus
 }

@@ -104,7 +104,7 @@ class SherfObservation(C.Structure):
 
 
 EXPORTS = ['sherf_render_backward_after_forward', 'sherf_sparse_encoder_train_scratch_bytes', 'sherf_sparse_encode_train', 'sherf_sparse_encode_backward', 'sherf_prepare_observation_backward', 'sherf_backward_scratch_bytes', 'sherf_render_backward', 'sherf_smpl_vertices', 'sherf_count_survivors', 'sherf_observation_scratch_bytes', 'sherf_prepare_observation', 'sherf_debug_set_trace', 'sherf_sparse_encoder_scratch_bytes', 'sherf_sparse_encode', 'sherf_generate_rays', 'sherf_debug_sample_importance', 'sherf_debug_linear', 'sherf_scratch_bytes', 'sherf_render_forward', 'sherf_lbs_transforms', 'sherf_depth_range', 'sherf_last_error',
-           'sherf_abi_version', 'sherf_last_launch_count', 'sherf_last_importance_point_count', 'sherf_set_profiling', 'sherf_last_stage_ms', 'sherf_last_host_us']
+           'sherf_abi_version', 'sherf_last_launch_count', 'sherf_last_importance_point_count', 'sherf_set_profiling', 'sherf_last_stage_ms', 'sherf_last_host_us', 'sherf_nn_list_stats']
 
 _lib = None
 
@@ -187,6 +187,8 @@ def load():
     lib.sherf_set_profiling.argtypes = [C.c_int]
     lib.sherf_last_stage_ms.restype = C.c_float
     lib.sherf_last_stage_ms.argtypes = [C.c_int]
+    lib.sherf_nn_list_stats.restype = C.c_int
+    lib.sherf_nn_list_stats.argtypes = [C.POINTER(C.c_double)]
     lib.sherf_last_host_us.restype = C.c_float
     lib.sherf_last_host_us.argtypes = [C.c_int]
     if lib.sherf_abi_version() != ABI_VERSION:

@@ -18,6 +18,7 @@ static thread_local int64_t g_last_launches = 0;
 static thread_local int64_t g_last_fine_points = 0;
 static thread_local int g_profiling = 0;
 static thread_local float g_stage_ms[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+static thread_local FrameTables g_last_ft{};                // tables of the last forward (sherf_nn_list_stats)
 static thread_local float g_host_us[4] = {0, 0, 0, 0};   // host wall time of the last forward: issue until the P sync, waiting in the sync, issue of the point stages, total
 static inline double now_us() { return std::chrono::duration<double, std::micro>(std::chrono::steady_clock::now().time_since_epoch()).count(); }
 
@@ -29,6 +30,16 @@ void set_error(const char* fmt, ...) {
 }
 
 constexpr int kMaxCell = 1 << 18;
+
+bool nn_lists_enabled() {
+  const char* e = getenv("SHERF_NN_LEGACY");
+  return !(e && atoi(e) != 0);
+}
+int nn_list_cap() {
+  const char* e = getenv("SHERF_NN_LIST_CAP");
+  const int k = e ? atoi(e) : kNnlCap;
+  return k < 1 ? 1 : (k > kNnlCap ? kNnlCap : k);
+}
 // points per MLP chunk (activation buffers are sized for this); SHERF_CHUNK_CAP overrides it for tuning experiments
 static size_t chunk_cap_limit() {
   static size_t cap = 0;
@@ -95,6 +106,16 @@ static size_t carve(Arena& a, const SherfScene& sc, int N, int S, int SF, int V,
   ft.g3_verts = a.take<float4>(V);
   ft.g1_occ = a.take<unsigned char>(kMaxCell);
   ft.maxcell = kMaxCell;
+  ft.nnl_on = nn_lists_enabled() ? 1 : 0;
+  ft.nnl_cap = nn_list_cap();
+  ft.nnl_count = a.take<int>(4);
+  ft.nnl_cand = a.take<unsigned char>((size_t)kMaxCell * kNnlSub3);
+  for (int g = 0; g < 2; ++g) {
+    ft.nnl_slot[g] = a.take<int>(kMaxCell);
+    ft.nnl_slot_cell[g] = a.take<int>(kNnlSlots);
+    ft.nnl_len[g] = a.take<int>((size_t)kNnlSlots * kNnlSub3);
+    ft.nnl_ent[g] = a.take<float4>((size_t)kNnlSlots * kNnlSub3 * kNnlCap);
+  }
   L.lbs_joints = a.take<float>(kJoints * 3);
   L.lbs_pf = a.take<float>(kPoseFeat);
   L.planes_cl = a.take<float>((size_t)3 * sc.plane_ch * sc.plane_h * sc.plane_w);
@@ -234,6 +255,7 @@ static void fill_gather_params(GatherParams& G, const SherfRays& rays, const She
   G.point_sample = L.point_sample; G.point_vid = L.point_vid; G.p0 = 0; G.np = 0; G.dc = DevCount{nullptr, 0, 0};
   G.fc = L.ft.fc; G.T1 = L.ft.T1; G.T3 = L.ft.T3; G.g3_start = L.ft.g3_cell_start; G.g3_verts = L.ft.g3_verts;
   G.t_vertices = getenv("SHERF_KNN3_UNSEEDED") ? nullptr : frame.t_vertices;
+  G.nl3 = L.ft.lists(1);
   G.planes_cl = L.planes_cl; G.plane_h = scene.plane_h; G.plane_w = scene.plane_w;
   G.feat_cl = L.feat_cl; G.feat_h = scene.feat_h; G.feat_w = scene.feat_w; G.feat_ch = scene.feat_ch;
   G.img = scene.obs_img; G.img_h = scene.img_h; G.img_w = scene.img_w;
@@ -298,6 +320,31 @@ int64_t sherf_last_importance_point_count(void) { return g_last_fine_points; }
 void sherf_set_profiling(int enabled) { g_profiling = enabled; }
 float sherf_last_stage_ms(int stage) { return (stage >= 0 && stage < 8) ? g_stage_ms[stage] : 0.f; }
 float sherf_last_host_us(int part) { return (part >= 0 && part < 4) ? g_host_us[part] : 0.f; }
+
+int sherf_nn_list_stats(double* out) {
+  if (!out || !g_last_ft.nnl_on) { set_error("the last forward on this thread built no candidate lists"); return SHERF_E_INVALID; }
+  const FrameTables& ft = g_last_ft;
+  SHERF_CUDA_OK(cudaDeviceSynchronize());
+  int cnt[4];
+  SHERF_CUDA_OK(cudaMemcpy(cnt, ft.nnl_count, sizeof(cnt), cudaMemcpyDeviceToHost));
+  out[0] = cnt[2];
+  std::vector<int> len((size_t)kNnlSlots * kNnlSub3);
+  for (int g = 0; g < 2; ++g) {
+    const int nsub = (cnt[g] < kNnlSlots ? cnt[g] : kNnlSlots) * kNnlSub3;
+    SHERF_CUDA_OK(cudaMemcpy(len.data(), ft.nnl_len[g], sizeof(int) * (size_t)nsub, cudaMemcpyDeviceToHost));
+    double sum = 0.0, mx = 0.0, over = 0.0;
+    for (int i = 0; i < nsub; ++i) {
+      if (len[i] < 0) over += 1.0;
+      else { sum += len[i]; mx = len[i] > mx ? len[i] : mx; }
+    }
+    out[1 + 4 * g] = nsub;
+    out[2 + 4 * g] = nsub > over ? sum / (nsub - over) : 0.0;
+    out[3 + 4 * g] = mx;
+    out[4 + 4 * g] = nsub ? over / nsub : 0.0;
+  }
+  out[9] = ft.nnl_cap;
+  return SHERF_OK;
+}
 
 size_t sherf_scratch_bytes(const SherfScene* scene, int32_t n_rays, int32_t n_samples, int32_t n_importance, int32_t n_verts) {
   if (!scene || n_rays <= 0 || n_samples < 2 || n_importance < 0 || n_verts <= 0) return 0;
@@ -571,6 +618,7 @@ int sherf_render_forward(const SherfSmplModel* smpl, const SherfFrame* frame, co
   }
   tm.finish();
   g_last_launches = g_launches.n;
+  g_last_ft = L.ft;
   { const double t_exit = now_us(); g_host_us[0] = (float)(t_sync0 - t_enter); g_host_us[1] = (float)(t_sync1 - t_sync0); g_host_us[2] = (float)(t_exit - t_sync1); g_host_us[3] = (float)(t_exit - t_enter); }
   return SHERF_OK;
 }
@@ -686,6 +734,9 @@ static int render_backward_impl(const SherfSmplModel* smpl, const SherfFrame* fr
     carve_bwd_chunk(B.chunk, B.bcap, bc);
     GatherParams G;
     fill_gather_params(G, *rays, *frame, *scene, L);
+    // the candidate lists in the arena are those of whichever forward ran on it last (with or without lists): the re-gather takes the
+    // grid search, which picks the same vertices
+    G.nl3 = NnLists{nullptr, nullptr, nullptr, nullptr};
     for (int64_t p0 = 0; p0 < P; p0 += B.bcap) {
       const int np = (int)((P - p0 < B.bcap) ? (P - p0) : B.bcap);
       RC(run_backward_chunk(*weights, pw, cw, cbw, gw, G, bc, np, p0, L.rgb, B.dsig, B.drgb, st));

@@ -22,6 +22,46 @@ struct GridDesc {
   int ncell;
 };
 
+// Candidate lists of the exact nearest-vertex searches.  Every coarse cell that has a vertex in its 27-neighbourhood gets a slot (up to
+// kNnlSlots per grid); each of its kNnlSub^3 sub-cells B holds up to kNnlCap vertices: every v with dmin(B, v) <= U(B) = d(centre(B), v*)
+// + half-diagonal(B) for a vertex v* near the centre (and, in the cull grid, dmin(B, v) < 5 cm), both with a conservative slack.  The
+// nearest vertex of any q in B and every vertex tied with it satisfy that test, so the lexicographic (d2, id) minimum over the list is
+// the global one.  Queries without a list (no slot, more than the capacity) take the grid search.
+constexpr int kNnlSub = 2;
+constexpr int kNnlSub3 = kNnlSub * kNnlSub * kNnlSub;
+constexpr int kNnlCap = 64;
+constexpr int kNnlSlots = 6144;
+
+struct NnLists {
+  const int* slot;      // [maxcell] coarse cell -> slot; -1: no vertex in its 27-neighbourhood, -2: occupied but no slot left
+  const int* len;       // [kNnlSlots * kNnlSub3] list length of a sub-cell, -1: more than the capacity
+  const float4* ent;    // [kNnlSlots * kNnlSub3][kNnlCap] (x, y, z, id bits)
+  const unsigned char* cand;   // cull grid only, [maxcell * kNnlSub3]: 0 = an empty list or no vertex in the 27-neighbourhood
+};
+
+// Coarse cell (grid_coord's) and sub-cell of q; false outside the grid.  The sub-cell is the fractional part of the same grid
+// coordinate (t - floor(t) and the power-of-two scale are exact), so q lies in the sub-cell up to the rounding of t.
+__device__ __forceinline__ bool nnl_cell(const GridDesc& g, float qx, float qy, float qz, int& cell, int& sub) {
+  const float tx = (qx - g.origin[0]) * g.inv_cell, ty = (qy - g.origin[1]) * g.inv_cell, tz = (qz - g.origin[2]) * g.inv_cell;
+  const int cx = (int)floorf(tx), cy = (int)floorf(ty), cz = (int)floorf(tz);
+  if (cx < 0 || cx >= g.dim[0] || cy < 0 || cy >= g.dim[1] || cz < 0 || cz >= g.dim[2]) return false;
+  cell = (cz * g.dim[1] + cy) * g.dim[0] + cx;
+  const int sx = min((int)((tx - (float)cx) * (float)kNnlSub), kNnlSub - 1);
+  const int sy = min((int)((ty - (float)cy) * (float)kNnlSub), kNnlSub - 1);
+  const int sz = min((int)((tz - (float)cz) * (float)kNnlSub), kNnlSub - 1);
+  sub = (sz * kNnlSub + sy) * kNnlSub + sx;
+  return true;
+}
+
+// List index (slot * kNnlSub3 + sub-cell) of the sub-cell that holds q, or -1 (q outside the grid), -2 (no vertex in the coarse cell's
+// 27-neighbourhood), -3 (occupied coarse cell without a slot)
+__device__ __forceinline__ int nnl_index(const GridDesc& g, const int* __restrict__ slot, float qx, float qy, float qz) {
+  int cell, sub;
+  if (!nnl_cell(g, qx, qy, qz, cell, sub)) return -1;
+  const int sl = slot[cell];
+  return sl < 0 ? sl - 1 : sl * kNnlSub3 + sub;
+}
+
 // Per-vertex piecewise-affine warp record.  Blend weights come from the single nearest vertex
 // (renderer.py:565,628), so the blended LBS matrices depend on the vertex id only.
 //   p  = Rinv * (p - t);  d = Rinv * d
@@ -136,7 +176,22 @@ struct FrameTables {           // device pointers carved out of the scratch aren
   float4* g3_verts;
   unsigned char* g1_occ;       // [maxcell] 27-neighbourhood occupancy
   int maxcell;
+  // candidate lists of the cull grid (0) and of the canonical grid (1); nnl_on = 0 (or null buffers): the grid searches only
+  int nnl_on;
+  int nnl_cap;                 // list capacity used by the build (<= kNnlCap)
+  int* nnl_slot[2];            // [maxcell]
+  int* nnl_slot_cell[2];       // [kNnlSlots] slot -> coarse cell
+  int* nnl_count;              // [4] slots taken per grid, cull candidates of the last cull
+  int* nnl_len[2];             // [kNnlSlots * kNnlSub3]
+  float4* nnl_ent[2];          // [kNnlSlots * kNnlSub3 * kNnlCap]
+  unsigned char* nnl_cand;     // [maxcell * kNnlSub3] candidate byte per sub-cell of the cull grid
+  NnLists lists(int g) const {
+    return nnl_on ? NnLists{nnl_slot[g], nnl_len[g], nnl_ent[g], g == 0 ? nnl_cand : nullptr} : NnLists{nullptr, nullptr, nullptr, nullptr};
+  }
 };
+// SHERF_NN_LEGACY=1: grid searches only; SHERF_NN_LIST_CAP=k: list capacity k (1..kNnlCap), read on every call
+bool nn_lists_enabled();
+int nn_list_cap();
 
 int run_prologue_frame(const SherfFrame& frame, const FrameTables& ft, cudaStream_t st);
 int run_prologue_cull(const SherfSmplModel& smpl, const SherfFrame& frame, const SherfRays& rays, const SherfOptions& opts,

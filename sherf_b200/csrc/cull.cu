@@ -1,5 +1,6 @@
 // Stage 1: sample points along rays, exact nearest posed-vertex search within the 5 cm cull radius
-// (uniform grid, 27-cell neighbourhood), ordered compaction of the survivors.
+// (per-sub-cell candidate lists, common.cuh: NnLists; uniform grid, 27-cell neighbourhood where a sub-cell has no list), ordered
+// compaction of the survivors.
 // Replaces renderer.py:299-321 (sample_stratified, SMPL-space transform, knn_points #1, mask, boolean-index
 // compaction).  Index bookkeeping is bit-exact against oracle/port.py (see its header for the rounding order).
 #include "common.cuh"
@@ -27,9 +28,11 @@ __device__ __forceinline__ void nn_27(const GridDesc& g, const int* __restrict__
 
 // The cull runs in two kernels so that the nearest-vertex search is load balanced: in a one-warp-per-ray formulation only the lanes
 // whose sample falls into an occupied cell search (7.6 of 32 on average at 512x512x64, profiles/r1_q), the rest of the warp idles.
-//   k_cull_candidates : one warp per ray, lane per sample: depth -> SMPL-space query -> grid cell -> occupancy byte; samples in
-//                       occupied cells are appended to a candidate queue (one atomicAdd per warp pass), all others get vid = -1
-//   k_cull_search     : one thread per candidate: exact 27-cell search, 5 cm test, per-ray survivor count (atomicAdd)
+//   k_cull_candidates : one warp per ray, lane per sample: depth -> SMPL-space query -> grid cell -> occupancy byte (with lists: the
+//                       sub-cell's candidate byte); candidates are appended to a queue (one atomicAdd per warp pass), all others get
+//                       vid = -1
+//   k_cull_search     : one thread per candidate: exact search over the sub-cell's list (27-cell search without one), 5 cm test,
+//                       per-ray survivor count (atomicAdd)
 // Candidates of a ray are contiguous in the queue, so neighbouring threads search neighbouring cells (similar trip counts).
 // Both kernels derive q with the same exactly-rounded operations, so the result is bit-identical to the single-kernel form.
 __device__ __forceinline__ void cull_query(const FrameConst& fc, const float* __restrict__ origins, const float* __restrict__ dirs, int n,
@@ -46,7 +49,7 @@ __global__ void __launch_bounds__(256) k_cull_candidates(const float* __restrict
                                                          const FrameConst* __restrict__ fcp, const unsigned char* __restrict__ occ,
                                                          const float* __restrict__ depths, int* __restrict__ sample_vid,
                                                          int* __restrict__ ray_count, int* __restrict__ queue, int* __restrict__ queue_count,
-                                                         int write_all) {
+                                                         int write_all, const NnLists nl) {
   __shared__ FrameConst fc;
   for (int i = threadIdx.x; i < (int)(sizeof(FrameConst) / 4); i += blockDim.x) ((int*)&fc)[i] = ((const int*)fcp)[i];
   __syncthreads();
@@ -93,10 +96,16 @@ __global__ void __launch_bounds__(256) k_cull_candidates(const float* __restrict
       if (t < t0 || t > t1) { sample_vid[(size_t)n * S + i] = -1; }
       else {
       cull_query(fc, origins, dirs, n, t, q);
-      const int cx = grid_coord(q[0], g.origin[0], g.inv_cell, g.dim[0]);
-      const int cy = grid_coord(q[1], g.origin[1], g.inv_cell, g.dim[1]);
-      const int cz = grid_coord(q[2], g.origin[2], g.inv_cell, g.dim[2]);
-      cand = cx >= 0 && cx < g.dim[0] && cy >= 0 && cy < g.dim[1] && cz >= 0 && cz < g.dim[2] && occ[(cz * g.dim[1] + cy) * g.dim[0] + cx];
+      if (nl.cand) {
+        // sub-cell byte: 0 for an empty cull list (no vertex within 5 cm of the sub-cell) as for an unoccupied coarse cell
+        int cell, sub;
+        cand = nnl_cell(g, q[0], q[1], q[2], cell, sub) && nl.cand[cell * kNnlSub3 + sub];
+      } else {
+        const int cx = grid_coord(q[0], g.origin[0], g.inv_cell, g.dim[0]);
+        const int cy = grid_coord(q[1], g.origin[1], g.inv_cell, g.dim[1]);
+        const int cz = grid_coord(q[2], g.origin[2], g.inv_cell, g.dim[2]);
+        cand = cx >= 0 && cx < g.dim[0] && cy >= 0 && cy < g.dim[1] && cz >= 0 && cz < g.dim[2] && occ[(cz * g.dim[1] + cy) * g.dim[0] + cx];
+      }
       if (!cand) sample_vid[(size_t)n * S + i] = -1;
       }
     }
@@ -110,29 +119,45 @@ __global__ void __launch_bounds__(256) k_cull_candidates(const float* __restrict
   }
 }
 
-__global__ void __launch_bounds__(256) k_cull_search(const float* __restrict__ origins, const float* __restrict__ dirs,
+// (256, 4): without a minimum occupancy ptxas capped the list form at 32 registers and spilled 128 bytes per thread
+__global__ void __launch_bounds__(256, 4) k_cull_search(const float* __restrict__ origins, const float* __restrict__ dirs,
                                                      const float* __restrict__ nearv, const float* __restrict__ farv, int S,
                                                      const FrameConst* __restrict__ fcp, const int* __restrict__ cell_start,
                                                      const float4* __restrict__ gv, float thr, const float* __restrict__ depths,
                                                      const int* __restrict__ queue, const int* __restrict__ queue_count,
-                                                     int* __restrict__ sample_vid, int* __restrict__ ray_count) {
+                                                     int* __restrict__ sample_vid, int* __restrict__ ray_count, const NnLists nl,
+                                                     int* __restrict__ cand_out) {
   __shared__ FrameConst fc;
   for (int i = threadIdx.x; i < (int)(sizeof(FrameConst) / 4); i += blockDim.x) ((int*)&fc)[i] = ((const int*)fcp)[i];
   __syncthreads();
   const GridDesc& g = fc.g1;
   const int count = *queue_count;
+  if (cand_out && blockIdx.x == 0 && threadIdx.x == 0) *cand_out = count;
   for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < count; j += gridDim.x * blockDim.x) {
     const int s = queue[j];
     const int n = s / S, i = s - n * S;
     const float t = depths ? depths[s] : sample_depth(nearv[n], farv[n], i, S);
     float q[3];
     cull_query(fc, origins, dirs, n, t, q);
-    const int cx = grid_coord(q[0], g.origin[0], g.inv_cell, g.dim[0]);
-    const int cy = grid_coord(q[1], g.origin[1], g.inv_cell, g.dim[1]);
-    const int cz = grid_coord(q[2], g.origin[2], g.inv_cell, g.dim[2]);
     float best = 3.0e38f;
     int bid = 0x7fffffff;
-    nn_27(g, cell_start, gv, q[0], q[1], q[2], cx, cy, cz, best, bid);
+    const float qx = q[0], qy = q[1], qz = q[2];
+    const int li = nl.slot ? nnl_index(g, nl.slot, qx, qy, qz) : -1;
+    const int ln = li >= 0 ? nl.len[li] : -1;
+    if (ln >= 0) {
+      const float4* e = nl.ent + (size_t)li * kNnlCap;
+      for (int k = 0; k < ln; ++k) {
+        const float4 v = e[k];
+        const float d2 = dist2_xyz(qx, qy, qz, v.x, v.y, v.z);
+        const int id = __float_as_int(v.w);
+        if (d2 < best || (d2 == best && id < bid)) { best = d2; bid = id; }
+      }
+    } else {                                 // no list (occupied cell without a slot, overflowing sub-cell): the grid search
+      const int cx = grid_coord(q[0], g.origin[0], g.inv_cell, g.dim[0]);
+      const int cy = grid_coord(q[1], g.origin[1], g.inv_cell, g.dim[1]);
+      const int cz = grid_coord(q[2], g.origin[2], g.inv_cell, g.dim[2]);
+      nn_27(g, cell_start, gv, qx, qy, qz, cx, cy, cz, best, bid);
+    }
     const int vid = best < thr ? bid : -1;
     sample_vid[s] = vid;
     if (vid >= 0) atomicAdd(&ray_count[n], 1);
@@ -232,10 +257,10 @@ int run_cull(const SherfRays& rays, int S, const float* depths, const FrameTable
   int* queue_count = reinterpret_cast<int*>(total_dev);
   SHERF_CUDA_OK(cudaMemsetAsync(queue_count, 0, sizeof(int), st));
   k_cull_candidates<<<ceil_div(N, 8), 256, 0, st>>>(rays.origins, rays.dirs, rays.near_, rays.far_, N, S, ft.fc, ft.g1_occ, depths,
-                                                    sample_vid, ray_count, queue, queue_count, write_all);
+                                                    sample_vid, ray_count, queue, queue_count, write_all, ft.lists(0));
   SHERF_LAUNCH_CHECK();
   k_cull_search<<<148 * 8, 256, 0, st>>>(rays.origins, rays.dirs, rays.near_, rays.far_, S, ft.fc, ft.g1_cell_start, ft.g1_verts, thr, depths,
-                                         queue, queue_count, sample_vid, ray_count);
+                                         queue, queue_count, sample_vid, ray_count, ft.lists(0), ft.nnl_on ? ft.nnl_count + 2 : nullptr);
   SHERF_LAUNCH_CHECK();
   RC_SCAN(run_exclusive_scan(ray_count, N, block_sums, ray_start, total_dev, st));
   k_compact<<<ceil_div(N, 8), 256, 0, st>>>(sample_vid, ray_start, N, S, point_sample, point_vid);

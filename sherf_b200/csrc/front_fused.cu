@@ -85,9 +85,27 @@ __device__ __forceinline__ void fr_grp_lexmin(float& d, int& id) {      // over 
   }
 }
 
-// exact K=1 search over the canonical vertices seeded by the nearest posed vertex (gather.cu: nn_seeded8), 4 lanes per point
+// exact K=1 search over the canonical vertices, 4 lanes per point: over the candidate list of the point's sub-cell (lane l4 takes entries
+// l4, l4 + 4, ...), or, where the sub-cell has no list, over the grid cells within the distance of the seed, the nearest posed vertex
+// (gather.cu: nn_seeded8)
 __device__ __forceinline__ int fr_nn_seeded4(const GridDesc& g, const int* __restrict__ cell_start, const float4* __restrict__ gv,
-                                             const float* __restrict__ t_vertices, float qx, float qy, float qz, int l4, int seed) {
+                                             const NnLists& nl, const float* __restrict__ t_vertices, float qx, float qy, float qz, int l4,
+                                             int seed) {
+  const int li = nl.slot ? nnl_index(g, nl.slot, qx, qy, qz) : -1;
+  const int ln = li >= 0 ? nl.len[li] : -1;
+  if (ln > 0) {
+    float best = 3.0e38f;
+    int bid = 0x7fffffff;
+    const float4* e = nl.ent + (size_t)li * kNnlCap;
+    for (int k = l4; k < ln; k += 4) {
+      const float4 v = e[k];
+      const float d2 = dist2_xyz(qx, qy, qz, v.x, v.y, v.z);
+      const int id = __float_as_int(v.w);
+      if (d2 < best || (d2 == best && id < bid)) { best = d2; bid = id; }
+    }
+    fr_grp_lexmin(best, bid);
+    return bid;
+  }
   float best = dist2_xyz(qx, qy, qz, t_vertices[seed * 3], t_vertices[seed * 3 + 1], t_vertices[seed * 3 + 2]);
   int bid = seed;
   const float rb = sqrtf(best) * 1.0001f + 1.0e-4f * g.cell;
@@ -206,7 +224,7 @@ __global__ void __launch_bounds__(fr::kThreads, 2) k_front_fused(const FrontArgs
       float cn[3] = {q[0], q[1], q[2]}, cdir[3] = {vd[0], vd[1], vd[2]};
       const int vid1 = P.point_vid[gp];
       if (!(a.knock & 8)) fr_apply_warp(P.T1 + vid1, cn, cdir, true);                  // target -> canonical   renderer.py:558-621
-      const int vid3 = (a.knock & 1) ? vid1 : fr_nn_seeded4(fc.g3, P.g3_start, P.g3_verts, P.t_vertices, cn[0], cn[1], cn[2], l4, vid1);
+      const int vid3 = (a.knock & 1) ? vid1 : fr_nn_seeded4(fc.g3, P.g3_start, P.g3_verts, P.nl3, P.t_vertices, cn[0], cn[1], cn[2], l4, vid1);
       float ps[3] = {cn[0], cn[1], cn[2]}, dummy[3] = {0.f, 0.f, 0.f};
       fr_apply_warp(P.T3 + vid3, ps, dummy, false);                                    // canonical -> observation   renderer.py:623-684
       float world[3], cam[3], pix[3];

@@ -350,8 +350,24 @@ __device__ __forceinline__ void grp_lexmin(float& d, int& id) {      // reduce o
 // ball of that radius need to be visited (typically 8-18 instead of 27 cells of 5 cm, and never a second, 125-cell round).  Any vertex
 // that beats or ties the seed lies inside the box [q - r, q + r], r = sqrt(d2_seed) (+ guard for the fp32 rounding of d2 and of the
 // cell coordinates), and the vertex cells are clamped exactly like the box, so the lexicographic (d2, id) minimum is unchanged.
-__device__ int nn_seeded8(const GridDesc& g, const int* __restrict__ cell_start, const float4* __restrict__ gv,
+// With candidate lists (common.cuh: NnLists) the 8 lanes scan the list of the point's sub-cell instead, where it has one.
+__device__ int nn_seeded8(const GridDesc& g, const int* __restrict__ cell_start, const float4* __restrict__ gv, const NnLists& nl,
                           const float* __restrict__ t_vertices, float qx, float qy, float qz, int l8, int seed) {
+  const int li = nl.slot ? nnl_index(g, nl.slot, qx, qy, qz) : -1;
+  const int ln = li >= 0 ? nl.len[li] : -1;
+  if (ln > 0) {
+    float best = 3.0e38f;
+    int bid = 0x7fffffff;
+    const float4* e = nl.ent + (size_t)li * kNnlCap;
+    for (int k = l8; k < ln; k += 8) {
+      const float4 v = e[k];
+      const float d2 = dist2_xyz(qx, qy, qz, v.x, v.y, v.z);
+      const int id = __float_as_int(v.w);
+      if (d2 < best || (d2 == best && id < bid)) { best = d2; bid = id; }
+    }
+    grp_lexmin(best, bid);
+    return bid;
+  }
   float best = dist2_xyz(qx, qy, qz, t_vertices[seed * 3], t_vertices[seed * 3 + 1], t_vertices[seed * 3 + 2]);
   int bid = seed;
   const float rb = sqrtf(best) * 1.0001f + 1.0e-4f * g.cell;
@@ -451,7 +467,7 @@ __global__ void __launch_bounds__(256) k_point_gather4(const GatherParams P) {
     rowvec_mat3(dray, fc.R_tgt, vd);
     float can[3] = {q[0], q[1], q[2]}, cdir[3] = {vd[0], vd[1], vd[2]};
     apply_warp(P.T1 + P.point_vid[gp], can, cdir, true);
-    const int vid3 = P.t_vertices ? nn_seeded8(fc.g3, P.g3_start, P.g3_verts, P.t_vertices, can[0], can[1], can[2], l8, P.point_vid[gp])
+    const int vid3 = P.t_vertices ? nn_seeded8(fc.g3, P.g3_start, P.g3_verts, BWD ? NnLists{nullptr, nullptr, nullptr, nullptr} : P.nl3, P.t_vertices, can[0], can[1], can[2], l8, P.point_vid[gp])
                                   : nn_unbounded8(fc.g3, P.g3_start, P.g3_verts, can[0], can[1], can[2], l8, active);
     float ps[3] = {can[0], can[1], can[2]}, dummy[3] = {0.f, 0.f, 0.f};
     apply_warp(P.T3 + vid3, ps, dummy, false);

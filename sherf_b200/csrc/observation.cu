@@ -207,7 +207,7 @@ int run_prepare_observation(const SherfSmplModel& smpl, const SherfObservation& 
   size_t off = 0;
   auto take = [&](size_t bytes) -> void* { off = (off + 255) & ~(size_t)255; void* p = base + off; off += bytes; return p; };
   { const size_t mis = ((size_t)base) & 255; if (mis) base += 256 - mis; }
-  FrameTables ft;
+  FrameTables ft{};
   ft.fc = (FrameConst*)take(sizeof(FrameConst));
   ObsConst* oc = (ObsConst*)take(sizeof(ObsConst));
   ft.A = (float*)take(sizeof(float) * 3 * kJoints * 16);
@@ -228,6 +228,7 @@ int run_prepare_observation(const SherfSmplModel& smpl, const SherfObservation& 
   ft.g3_verts = (float4*)take(sizeof(float4) * (size_t)V);
   ft.g1_occ = (unsigned char*)take(kMaxCell);
   ft.maxcell = kMaxCell;
+  ft.nnl_on = 0;                     // this path has no nearest-vertex queries
   unsigned char* vmask = vmask_out ? vmask_out : (unsigned char*)take(V);
 
   // the render path's per-vertex warp tables with the OBSERVATION pose in the "target" slot: T1[v] = observation SMPL space ->

@@ -276,8 +276,9 @@ __global__ void __launch_bounds__(256) k_verts_smpl(const float* __restrict__ ve
 // grid: the single-block form spent 190 us (profiles/r1_q: 55 % of its stalls on the 27 byte stores per vertex of the dilation,
 // the rest on serial passes over the cells by one SM) on the critical path in front of the cull.
 __global__ void __launch_bounds__(1024) k_grid_setup(const float* __restrict__ verts_smpl, const float* __restrict__ t_vertices, int V,
-                                                      int maxcell, float min_cell, FrameConst* fc, int g0) {
+                                                      int maxcell, float min_cell, FrameConst* fc, int g0, int* nslots) {
   const int g = g0 + blockIdx.x;
+  if (nslots && threadIdx.x == 0) nslots[g] = 0;              // list slots of this grid are counted by k_grid_occupancy
   const float* P = g == 0 ? verts_smpl : t_vertices;
   GridDesc* gd = g == 0 ? &fc->g1 : &fc->g3;
   const int tid = threadIdx.x, nt = blockDim.x;
@@ -351,10 +352,13 @@ __global__ void __launch_bounds__(256) k_grid_scatter(const float* __restrict__ 
   (g == 0 ? g1_verts : g3_verts)[pos] = make_float4(x, y, z, __int_as_float(v));
 }
 
-// occupancy byte of a cull-grid cell = "some vertex lies in its 27-neighbourhood" (cells of a row are contiguous in cell_start)
-__global__ void __launch_bounds__(256) k_grid_occupancy(const FrameConst* __restrict__ fc, const int* __restrict__ g1_start,
-                                                        unsigned char* __restrict__ occ) {
-  const GridDesc sg = fc->g1;
+// occupancy of a cell = "some vertex lies in its 27-neighbourhood" (cells of a row are contiguous in cell_start): the cull grid's byte
+// and, when the candidate lists are built, the list slot of the cell (nnl_slot / nnl_slot_cell, counted in *nslots, one atomic per warp)
+// and the cull grid's sub-cell candidate bytes (1 for every sub-cell of an occupied cell; k_nnl_build clears those with empty lists)
+__global__ void __launch_bounds__(256) k_grid_occupancy(const FrameConst* __restrict__ fc, int g, const int* __restrict__ start,
+                                                        unsigned char* __restrict__ occ, int* __restrict__ slot, int* __restrict__ slot_cell,
+                                                        int* __restrict__ nslots, unsigned char* __restrict__ cand) {
+  const GridDesc sg = g == 0 ? fc->g1 : fc->g3;
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= sg.ncell) return;
   const int x = c % sg.dim[0], t = c / sg.dim[0], y = t % sg.dim[1], z = t / sg.dim[1];
@@ -363,9 +367,126 @@ __global__ void __launch_bounds__(256) k_grid_occupancy(const FrameConst* __rest
   for (int zz = max(z - 1, 0); zz <= min(z + 1, sg.dim[2] - 1); ++zz)
     for (int yy = max(y - 1, 0); yy <= min(y + 1, sg.dim[1] - 1); ++yy) {
       const int row = (zz * sg.dim[1] + yy) * sg.dim[0];
-      any |= g1_start[row + x1 + 1] > g1_start[row + x0];
+      any |= start[row + x1 + 1] > start[row + x0];
     }
-  occ[c] = any ? 1 : 0;
+  if (occ) occ[c] = any ? 1 : 0;
+  if (cand) *reinterpret_cast<uint2*>(cand + (size_t)c * kNnlSub3) = any ? make_uint2(0x01010101u, 0x01010101u) : make_uint2(0u, 0u);
+  if (slot) {
+    const unsigned act = __activemask(), m = __ballot_sync(act, any);
+    const int lane = threadIdx.x & 31, leader = __ffs(act) - 1;
+    int base = 0;
+    if (lane == leader && m) base = atomicAdd(nslots, __popc(m));
+    base = __shfl_sync(act, base, leader);
+    int s = -1;
+    if (any) {
+      s = base + __popc(m & ((1u << lane) - 1u));
+      if (s < kNnlSlots) slot_cell[s] = c;
+      else s = -2;
+    }
+    slot[c] = s;
+  }
+}
+
+// Candidate lists (common.cuh: NnLists), one warp per slotted coarse cell, all kNnlSub^3 = 8 sub-cells at once (the cell's vertex
+// neighbourhood is read once).  Box B = the sub-cell grown by 1e-4 of a coarse cell on every side (covers the rounding of the queries'
+// grid coordinates).  U = d(centre, v*) + half-diagonal(B) with v* the vertex of the 27-neighbourhood nearest to the centre; the list
+// takes every v with dmin(B, v) <= lim = U (1 + 1e-4) + 1e-4 cell, lim capped at `cut` in the cull grid (5 cm with the same slack).
+// Vertices with dmin(B, v) <= lim lie in the (2r+1)^3 block of cells around B when lim < r cells; r = 1 or 2, beyond that (and beyond
+// `cap` entries) the sub-cell is marked -1 and its queries take the grid search.  cand (cull grid): 0 for the sub-cells with empty lists.
+__global__ void __launch_bounds__(256) k_nnl_build(const FrameConst* __restrict__ fc, int g, const int* __restrict__ start,
+                                                   const float4* __restrict__ gv, const int* __restrict__ slot_cell,
+                                                   const int* __restrict__ nslots, int cap, float cut, int* __restrict__ len,
+                                                   float4* __restrict__ ent, unsigned char* __restrict__ cand) {
+  static_assert(kNnlSub == 2, "one bit per axis selects the sub-cell");
+  const GridDesc sg = g == 0 ? fc->g1 : fc->g3;
+  const int lane = threadIdx.x & 31;
+  const int ns = min(*nslots, kNnlSlots);
+  const float f = sg.cell * 0.5f, eps = 1.0e-4f * sg.cell;
+  for (int sl = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; sl < ns; sl += (gridDim.x * blockDim.x) >> 5) {
+    const int c = slot_cell[sl];
+    const int cx = c % sg.dim[0], t = c / sg.dim[0], cy = t % sg.dim[1], cz = t / sg.dim[1];
+    const int cc[3] = {cx, cy, cz};
+    float lo[3][2], hi[3][2], ctr[3][2];                     // per axis and sub-cell coordinate
+#pragma unroll
+    for (int k = 0; k < 3; ++k)
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        lo[k][h] = sg.origin[k] + (float)cc[k] * sg.cell + (float)h * f - eps;
+        hi[k][h] = lo[k][h] + f + 2.f * eps;
+        ctr[k][h] = 0.5f * (lo[k][h] + hi[k][h]);
+      }
+    // v* of every sub-cell: nearest vertex of the 27-neighbourhood to its centre (the coarse cell is occupied, so there is one)
+    float dc[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) dc[i] = 3.0e38f;
+    for (int zz = max(cz - 1, 0); zz <= min(cz + 1, sg.dim[2] - 1); ++zz)
+      for (int yy = max(cy - 1, 0); yy <= min(cy + 1, sg.dim[1] - 1); ++yy) {
+        const int row = (zz * sg.dim[1] + yy) * sg.dim[0];
+        const int b = start[row + max(cx - 1, 0)], e = start[row + min(cx + 1, sg.dim[0] - 1) + 1];
+        for (int k = b + lane; k < e; k += 32) {
+          const float4 v = gv[k];
+          float d[3][2];
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            d[0][h] = (v.x - ctr[0][h]) * (v.x - ctr[0][h]);
+            d[1][h] = (v.y - ctr[1][h]) * (v.y - ctr[1][h]);
+            d[2][h] = (v.z - ctr[2][h]) * (v.z - ctr[2][h]);
+          }
+#pragma unroll
+          for (int i = 0; i < 8; ++i) dc[i] = fminf(dc[i], d[0][i & 1] + d[1][(i >> 1) & 1] + d[2][i >> 2]);
+        }
+      }
+    float lim2[8];
+    int rmax = 0, rbits = 0;                                   // bit i: sub-cell i has a usable bound
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      float x = dc[i];
+      for (int o = 16; o > 0; o >>= 1) x = fminf(x, __shfl_xor_sync(0xffffffffu, x, o));
+      float lim = (sqrtf(x) + 1.7320508f * (0.5f * f + eps)) * 1.0001f + eps;
+      if (cut > 0.f) lim = fminf(lim, cut);
+      const int r = lim < 0.999f * sg.cell ? 1 : (lim < 1.999f * sg.cell ? 2 : 0);
+      rmax = max(rmax, r);
+      rbits |= r > 0 ? 1 << i : 0;
+      lim2[i] = r > 0 ? lim * lim : -1.f;
+    }
+    int n[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) n[i] = 0;
+    float4* out = ent + (size_t)sl * kNnlSub3 * kNnlCap;
+    for (int zz = max(cz - rmax, 0); zz <= min(cz + rmax, sg.dim[2] - 1); ++zz)
+      for (int yy = max(cy - rmax, 0); yy <= min(cy + rmax, sg.dim[1] - 1); ++yy) {
+        const int row = (zz * sg.dim[1] + yy) * sg.dim[0];
+        const int b = start[row + max(cx - rmax, 0)], e = start[row + min(cx + rmax, sg.dim[0] - 1) + 1];
+        for (int k0 = b; k0 < e; k0 += 32) {
+          const int k = k0 + lane;
+          const float4 v = k < e ? gv[k] : make_float4(3.0e38f, 3.0e38f, 3.0e38f, 0.f);
+          float o[3][2];
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            const float ox = fmaxf(fmaxf(lo[0][h] - v.x, v.x - hi[0][h]), 0.f);
+            const float oy = fmaxf(fmaxf(lo[1][h] - v.y, v.y - hi[1][h]), 0.f);
+            const float oz = fmaxf(fmaxf(lo[2][h] - v.z, v.z - hi[2][h]), 0.f);
+            o[0][h] = ox * ox; o[1][h] = oy * oy; o[2][h] = oz * oz;
+          }
+#pragma unroll
+          for (int i = 0; i < 8; ++i) {
+            const bool take = k < e && o[0][i & 1] + o[1][(i >> 1) & 1] + o[2][i >> 2] <= lim2[i];
+            const unsigned m = __ballot_sync(0xffffffffu, take);
+            const int pos = n[i] + __popc(m & ((1u << lane) - 1u));
+            if (take && pos < cap) out[i * kNnlCap + pos] = v;
+            n[i] += __popc(m);
+          }
+        }
+      }
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      if (lane == i) {
+        const int l = ((rbits >> i) & 1) && n[i] <= cap ? n[i] : -1;
+        len[sl * kNnlSub3 + i] = l;
+        if (cand) cand[(size_t)c * kNnlSub3 + i] = l != 0;
+      }
+    }
+  }
 }
 
 // global min / max over all sample depths = over rays of {t_0, t_{S-1}} (t is monotone in i)   ray_marcher.py:57
@@ -415,7 +536,8 @@ int run_depth_range(const SherfRays& rays, FrameConst* fc, cudaStream_t st) {
 static int build_grid(int g, const SherfFrame& fr, const FrameTables& ft, int V, cudaStream_t st) {
   int* counts = ft.g_cursor + (size_t)g * ft.maxcell;
   int* bsums = ft.g_block_sums + (size_t)g * (ft.maxcell / 1024 + 2);
-  k_grid_setup<<<1, 1024, 0, st>>>(ft.verts_smpl, fr.t_vertices, V, ft.maxcell, 0.0505f, ft.fc, g);
+  const bool lists = ft.nnl_on != 0;
+  k_grid_setup<<<1, 1024, 0, st>>>(ft.verts_smpl, fr.t_vertices, V, ft.maxcell, 0.0505f, ft.fc, g, lists ? ft.nnl_count : nullptr);
   SHERF_LAUNCH_CHECK();
   SHERF_CUDA_OK(cudaMemsetAsync(counts, 0, sizeof(int) * (size_t)ft.maxcell, st));
   k_grid_count<<<dim3(ceil_div(V, 256), 1), 256, 0, st>>>(ft.verts_smpl, fr.t_vertices, V, ft.fc, ft.g_cursor, ft.maxcell, g);
@@ -426,8 +548,18 @@ static int build_grid(int g, const SherfFrame& fr, const FrameTables& ft, int V,
   k_grid_scatter<<<dim3(ceil_div(V, 256), 1), 256, 0, st>>>(ft.verts_smpl, fr.t_vertices, V, ft.fc, ft.g_cursor, ft.maxcell, ft.g1_cell_start,
                                                            ft.g3_cell_start, ft.g1_verts, ft.g3_verts, g);
   SHERF_LAUNCH_CHECK();
-  if (g == 0) {
-    k_grid_occupancy<<<ceil_div(ft.maxcell, 256), 256, 0, st>>>(ft.fc, ft.g1_cell_start, ft.g1_occ);
+  if (g == 0 || lists) {
+    k_grid_occupancy<<<ceil_div(ft.maxcell, 256), 256, 0, st>>>(ft.fc, g, g == 0 ? ft.g1_cell_start : ft.g3_cell_start, g == 0 ? ft.g1_occ : nullptr,
+                                                                lists ? ft.nnl_slot[g] : nullptr, ft.nnl_slot_cell[g], ft.nnl_count + g,
+                                                                lists && g == 0 ? ft.nnl_cand : nullptr);
+    SHERF_LAUNCH_CHECK();
+  }
+  if (lists) {
+    // the cull lists keep only what can pass the cull's 5 cm test (run_cull: d2 < 0.05^2 in fp32), with the same slack as the bound
+    const float cut = g == 0 ? 0.05f * 1.0001f + 1.0e-5f : 0.f;
+    k_nnl_build<<<148 * 8, 256, 0, st>>>(ft.fc, g, g == 0 ? ft.g1_cell_start : ft.g3_cell_start, g == 0 ? ft.g1_verts : ft.g3_verts,
+                                         ft.nnl_slot_cell[g], ft.nnl_count + g, ft.nnl_cap, cut, ft.nnl_len[g], ft.nnl_ent[g],
+                                         g == 0 ? ft.nnl_cand : nullptr);
     SHERF_LAUNCH_CHECK();
   }
   return SHERF_OK;

@@ -27,6 +27,7 @@ struct GatherParams {
   const VertexWarp *T1, *T3;
   const int* g3_start; const float4* g3_verts;
   const float* t_vertices;   // [V,3] canonical vertices (seed of the knn #3 search); NULL: unseeded doubling-box search
+  NnLists nl3;               // candidate lists of the canonical grid (slot == NULL: none)
   // channels-last features
   const float* planes_cl; int plane_h, plane_w;            // [3][H][W][32]
   const float* feat_cl; int feat_h, feat_w, feat_ch;       // [fh][fw][64]
